@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py - headline benchmark of the ProMP hot path on B200.
 
-    python bench.py --gpus N --steps K --warmup W [--workload point|cheetah] [--impl reference]
+    python bench.py --gpus N --steps K --warmup W [--workload point|cheetah] [--impl reference] [--dump-outputs DIR]
 
 A "step" is ONE FULL META-ITERATION of the hot path over one batch of synthetic tasks
 (BASELINE.json configs[1]: MetaPointEnvCorner, 40 tasks x 20 envs x H=100, ProMP, 2x(64) Gaussian MLP):
@@ -138,6 +138,27 @@ def build_stack(wl, reset_mode, task_shard=None, algo='promp', tasks=None, **tra
     return trainer
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+PHASE_OUTPUTS = ('obs', 'act', 'mean', 'log_std', 'rew', 'returns', 'adv', 'coeffs', 'stats')
+
+
+def dump_outputs(out_dir, policy, phases):
+    """Write what one timed meta-iteration hands its caller as out_dir/<name>.npy: the updated policy parameters (theta)
+    and, per sampling phase s, the trajectories, the policy's distribution parameters, returns, advantages, baseline
+    coefficients and path statistics (phase<s>_<name>).  Inputs are seeded, so two builds run with the same arguments can
+    be compared array by array."""
+    arrays = {'theta': policy.theta}
+    for s, ph in enumerate(phases):
+        arrays.update(('phase%d_%s' % (s, name), getattr(ph, name)) for name in PHASE_OUTPUTS)
+    arrays = {k: v.detach().cpu().numpy() for k, v in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise RuntimeError('--dump-outputs: %d bytes exceed the %d-byte limit' % (total, DUMP_LIMIT_BYTES))
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, k + '.npy'), a)
+
+
 class LaunchCounter(object):
     """Counts OUR kernel launches by wrapping the ctypes entry points (kernels per call from the .cu files)."""
     KERNELS = dict(promp_rollout=1, promp_env_step=1, promp_env_observe=1, promp_process_samples=1,
@@ -220,6 +241,7 @@ def run_gpu(args):
         torch.cuda.synchronize()
 
     def timed(trainer, log, n_warm, n_steps, step_fn=None):
+        """(device ms, wall ms, what the last timed step returned)"""
         run = step_fn if step_fn is not None else (lambda: trainer.train_iteration(0, log=log))
         for i in range(n_warm):
             run()
@@ -227,8 +249,9 @@ def run_gpu(args):
         a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         t0 = time.perf_counter()
         a.record()
-        for i in range(n_steps):
+        for i in range(n_steps - 1):
             run()
+        last = run()        # only the last result is kept: holding each one into the next step would double the eager buffers
         b.record()
         barrier()
         wall = time.perf_counter() - t0
@@ -236,7 +259,7 @@ def run_gpu(args):
         t = torch.tensor([ms, wall * 1e3], dtype=torch.float64, device='cuda')
         if world > 1:
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
-        return float(t[0]), float(t[1])
+        return float(t[0]), float(t[1]), last
 
     # ---- value: device-resident loop --------------------------------------------------------------
     np.random.seed(1)
@@ -244,15 +267,18 @@ def run_gpu(args):
     clocks = ClockSampler(local_rank) if rank == 0 else None
     use_graph = not args.no_graph       # N > 1: the all-reduce inside the graph is the P2P kernel (promp_allreduce_p2p)
     with LaunchCounter() as lc:
-        ms_eager, wall_eager = timed(tr_dev, False, args.warmup, args.steps)
+        ms_eager, wall_eager, last = timed(tr_dev, False, args.warmup, args.steps)
     launches = lc.count // (args.warmup + args.steps)
     if use_graph:
         # the same ~40 launches per meta-iteration captured once into a CUDA graph and replayed
         step_fn = tr_dev.capture_graph(warmup=2)
-        ms_dev, wall_dev = timed(tr_dev, False, args.warmup, args.steps, step_fn)
+        ms_dev, wall_dev, phases = timed(tr_dev, False, args.warmup, args.steps, step_fn)
     else:
         ms_dev, wall_dev = ms_eager, wall_eager
+        phases = [samples[0].phase for samples in last]
     clk = clocks.stop() if clocks else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, tr_dev.policy, phases)
     # ---- e2e: the default entry point of a run script - Trainer.train() - with host inputs / logged outputs ----------
     def timed_train(trainer, n_warm, n_steps):
         """Time n_steps meta-iterations of trainer.train() (device events + wall clock, max over ranks) after n_warm."""
@@ -285,7 +311,7 @@ def run_gpu(args):
                    'one CUDA-graph replay of the device part (captured automatically: fixed-horizon env, fixed KL coefficient), one D2H '
                    'of the logged scalars, logger.logkv of every reference key, logger.dumpkvs()')
     else:
-        ms_e2e, wall_e2e = timed(tr_e2e, True, args.warmup, args.steps)
+        ms_e2e, wall_e2e, _ = timed(tr_e2e, True, args.warmup, args.steps)
         h2d = 4 * (M * sd['task_dim'] + S * M * E * sd['state_dim'])
         d2h = S * (M * 8 * 8 + M * sd['act_dim'] * 4 + (2 * M * E * H * 4 * 2 if sd['env_kind'] == 2 else 0)) + 4 * (3 + S - 1)
         e2e_api = 'promp_b200.meta_trainer.Trainer.train_iteration(log=True), reset_mode=numpy'
@@ -293,7 +319,7 @@ def run_gpu(args):
     # inside the iteration get (adaptive KL coefficient, early-terminating envs, E-MAML)
     np.random.seed(1)
     tr_eager = build_stack(wl, 'numpy', shard, use_cuda_graph=False)
-    ms_e2e_eager, wall_e2e_eager = timed(tr_eager, True, args.warmup, args.steps)
+    ms_e2e_eager, wall_e2e_eager, _ = timed(tr_eager, True, args.warmup, args.steps)
 
     # ---- the other BASELINE.json configurations, measured in the same run (short): HalfCheetah surrogate (configs[2] per GPU =
     #      configs[4] at N = 8, weak scaling) and TRPO-MAML on PointEnv (configs[3]: 40 tasks in total, STRONG scaling)
@@ -707,7 +733,11 @@ def main():
     ap.add_argument('--no-extras', action='store_true', help='skip the short cheetah / TRPO-MAML measurements (other_configs)')
     ap.add_argument('--cpu-serial', action='store_true', help='CPU arm: single process on a 10-task sample instead of one worker process per task')
     ap.add_argument('--no-graph', action='store_true', help='time the device-resident loop eagerly instead of replaying a CUDA graph')
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='after the timed steps, write what the last timed meta-iteration computed as DIR/<name>.npy')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
     args.warmup = max(args.warmup, 3) if args.impl != 'reference' else max(args.warmup, 1)
     if args.impl == 'reference':
         run_reference(args)

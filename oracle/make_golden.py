@@ -574,20 +574,89 @@ def gen_baseline_known():
                         norm_adv=utils.normalize_advantages(x), pos_adv=utils.shift_advantages_to_positive(x))
 
 
+def gen_stack_tensor_dict_list():
+    """utils.stack_tensor_dict_list (utils/utils.py:144-159) on per-step info dicts with a nested dict: the trajectory
+    bookkeeping of the stepwise sampler.  The inputs are re-drawn by the test from the same seed."""
+    from meta_policy_search.utils import utils
+    rng = np.random.RandomState(0)
+    steps = [dict(mean=rng.randn(3), log_std=rng.randn(3), nested=dict(a=rng.randn(2), b=float(i))) for i in range(7)]
+    got = utils.stack_tensor_dict_list(steps)
+    np.savez_compressed(os.path.join(OUT, 'stack_tensor_dict_list.npz'), keys=np.asarray(sorted(got)),
+                        nested_keys=np.asarray(sorted(got['nested'])), mean=got['mean'], log_std=got['log_std'],
+                        nested_a=got['nested']['a'], nested_b=got['nested']['b'])
+
+
+def gen_trainer_protocol():
+    """What the UNMODIFIED reference Trainer (meta_trainer.py:59-152) asks of the objects it drives: the sequence of
+    method calls it makes on recording doubles (2 iterations, 1 inner step), and the TensorFlow names it uses, with
+    promp_b200/tf_shim imported as `tensorflow` (INTEGRATION.md section 1)."""
+    import importlib.util
+    import types
+    spec = importlib.util.spec_from_file_location(
+        'tensorflow', os.path.join(ROOT, 'promp_b200', 'tf_shim', 'tensorflow', '__init__.py'))
+    shim = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(shim)
+    tf_used, session_used, calls = set(), set(), []
+
+    class RecordingSession(shim.Session):
+        def __getattribute__(self, k):
+            if not k.startswith('_'):
+                session_used.add(k)
+            return object.__getattribute__(self, k)
+
+    class RecordingTF(types.ModuleType):
+        def __getattr__(self, k):
+            tf_used.add(k)
+            return RecordingSession if k == 'Session' else getattr(shim, k)
+
+    class Rec(object):
+        def __init__(self, name):
+            self._n = name
+
+        def __getattr__(self, k):
+            def f(*a, **kw):
+                calls.append(self._n + '.' + k)
+                if k == 'obtain_samples':
+                    return {0: [dict(x=1)], 1: [dict(x=2)]}
+                if k == 'process_samples':
+                    return ['samples']
+                return None
+            return f
+
+    saved = {k: sys.modules.pop(k) for k in ('tensorflow', 'meta_policy_search.meta_trainer') if k in sys.modules}
+    sys.modules['tensorflow'] = RecordingTF('tensorflow')
+    try:
+        from meta_policy_search.meta_trainer import Trainer
+    finally:
+        sys.modules.pop('tensorflow')
+        sys.modules.pop('meta_policy_search.meta_trainer', None)
+        sys.modules.update(saved)
+    sampler = Rec('sampler')
+    sampler.total_timesteps_sampled = 0
+    proc = Rec('proc')
+    proc.baseline = Rec('baseline')
+    Trainer(algo=Rec('algo'), env=Rec('env'), sampler=sampler, sample_processor=proc, policy=Rec('policy'), n_itr=2,
+            num_inner_grad_steps=1).train()
+    np.savez_compressed(os.path.join(OUT, 'trainer_protocol.npz'), calls=np.asarray(calls),
+                        tf_names=np.asarray(sorted(tf_used)), session_methods=np.asarray(sorted(session_used)))
+
+
 if __name__ == '__main__':
     _import_reference()
     os.makedirs(OUT, exist_ok=True)
     if len(sys.argv) > 1 and sys.argv[1] == 'tf_half_graph':      # python oracle/make_golden.py tf_half_graph [case ...]
         gen_tf_half_graph(only=sys.argv[2:] or None)
         sys.exit(0)
-    if len(sys.argv) > 1 and sys.argv[1] == 'trainer_run':
-        gen_trainer_run()
+    if len(sys.argv) > 1 and sys.argv[1] in ('trainer_run', 'stack_tensor_dict_list', 'trainer_protocol'):
+        globals()['gen_' + sys.argv[1]]()
         sys.exit(0)
     gen_point_corner_steps()
     gen_point_env_steps()
     gen_process_samples()
     gen_sampler_rollout()
     gen_baseline_known()
+    gen_stack_tensor_dict_list()
+    gen_trainer_protocol()
     gen_process_samples_ragged()
     gen_point_variants_steps()
     gen_tf_half_numpy_known()

@@ -175,44 +175,52 @@ def test_two_rank_gloo_sharding_and_allreduce():
 
 
 # ------------------------------------------------------------------ the reference's unchanged Trainer
-def test_reference_trainer_drives_promp_classes_unchanged():
-    """meta_policy_search/meta_trainer.py (unmodified, imported from /root/reference) runs against objects with
-    the promp_b200 interface, with promp_b200/tf_shim standing in for TensorFlow.  Needs the reference tree."""
-    if not os.path.isdir('/root/reference'):
-        pytest.skip("reference tree not present on this box")
-    code = r'''
-import sys, os
-root = %r
-sys.path.insert(0, os.path.join(root, 'promp_b200', 'tf_shim'))
-sys.path.insert(0, os.path.join(root, 'oracle', 'stubs'))
-sys.path.insert(0, '/root/reference')
-sys.path.insert(0, root)
-from meta_policy_search.meta_trainer import Trainer
-calls = []
-class Rec(object):
-    def __init__(self, name): self._n = name
-    def __getattr__(self, k):
-        def f(*a, **kw):
-            calls.append(self._n + '.' + k)
-            if k == 'obtain_samples': return {0: [dict(x=1)], 1: [dict(x=2)]}
-            if k == 'process_samples': return ['samples']
-            return None
-        return f
-sampler = Rec('sampler'); sampler.total_timesteps_sampled = 0
-proc = Rec('proc'); proc.baseline = Rec('baseline')
-tr = Trainer(algo=Rec('algo'), env=Rec('env'), sampler=sampler, sample_processor=proc, policy=Rec('policy'), n_itr=2,
-             num_inner_grad_steps=1)
-tr.train()
-want = ['sampler.update_tasks', 'policy.switch_to_pre_update', 'sampler.obtain_samples', 'proc.process_samples',
-        'env.log_diagnostics', 'policy.log_diagnostics', 'baseline.log_diagnostics', 'algo._adapt',
-        'sampler.obtain_samples', 'proc.process_samples', 'env.log_diagnostics', 'policy.log_diagnostics',
-        'baseline.log_diagnostics', 'algo.optimize_policy']
-assert calls[:len(want)] == want, calls
-assert calls.count('algo.optimize_policy') == 2
-print('reference trainer ok')
-''' % ROOT
-    r = subprocess.run([sys.executable, '-c', code], capture_output=True, text=True, timeout=240)
-    assert r.returncode == 0 and 'reference trainer ok' in r.stdout, r.stdout[-2000:] + r.stderr[-2000:]
+def test_reference_trainer_drives_promp_classes_unchanged(golden_dir):
+    """The driver protocol of meta_policy_search/meta_trainer.py (unmodified): tests/golden/trainer_protocol.npz holds the
+    method calls the reference Trainer makes on recording doubles over 2 iterations with one inner step, and the
+    TensorFlow names it uses with promp_b200/tf_shim imported as `tensorflow` (oracle/make_golden.py::gen_trainer_protocol).
+    promp_b200's Trainer must make the same calls in the same order (plus the sampler capability probe that decides on
+    CUDA-graph replay), and the shim must provide every name the reference Trainer takes from TensorFlow."""
+    import importlib.util
+    from promp_b200.meta_trainer import Trainer
+    from promp_b200.utils import logger
+    g = np.load(os.path.join(golden_dir, 'trainer_protocol.npz'))
+    calls = []
+
+    class Rec(object):
+        def __init__(self, name):
+            self._n = name
+
+        def __getattr__(self, k):
+            def f(*a, **kw):
+                calls.append(self._n + '.' + k)
+                if k == 'obtain_samples':
+                    return {0: [dict(x=1)], 1: [dict(x=2)]}
+                if k == 'process_samples':
+                    return ['samples']
+                return None
+            return f
+    sampler = Rec('sampler')
+    sampler.total_timesteps_sampled = 0
+    proc = Rec('proc')
+    proc.baseline = Rec('baseline')
+    logger.set_quiet(True)
+    Trainer(algo=Rec('algo'), env=Rec('env'), sampler=sampler, sample_processor=proc, policy=Rec('policy'), n_itr=2,
+            num_inner_grad_steps=1).train()
+    assert calls[0] == 'sampler._fused_ok', calls
+    assert calls[1:] == list(g['calls']), calls
+    spec = importlib.util.spec_from_file_location(
+        'tf_shim', os.path.join(ROOT, 'promp_b200', 'tf_shim', 'tensorflow', '__init__.py'))
+    tf = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(tf)
+    for name in g['tf_names']:
+        assert callable(getattr(tf, str(name), None)), name
+    sess = tf.Session()
+    for name in g['session_methods']:
+        assert callable(getattr(sess, str(name), None)), name
+    with sess.as_default() as s:
+        assert s is sess and s.run(tf.variables_initializer(tf.global_variables())) is None
+    sess.close()
 
 
 def test_logger_file_formats_and_snapshot_modes(tmp_path):
@@ -263,24 +271,20 @@ def test_ragged_phase_path_table():
     assert ph.obs.shape == (3, 56, 2) and float(ph.obs.abs().sum()) == 0.0       # padding rows start zeroed
 
 
-@pytest.mark.skipif(not os.path.isdir('/root/reference/meta_policy_search'), reason='reference tree not present')
-def test_path_stacking_matches_reference_utils():
+def test_path_stacking_matches_reference_utils(golden_dir):
     """Trajectory bookkeeping of the stepwise sampler (SURVEY row a8): per-step info dicts -> one dict of stacked arrays,
-    nested dicts included, exactly like utils.stack_tensor_dict_list (meta_policy_search/utils/utils.py) run from the
-    unmodified reference."""
-    import importlib.util
-    spec = importlib.util.spec_from_file_location('ref_utils', '/root/reference/meta_policy_search/utils/utils.py')
-    ref_utils = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(ref_utils)
+    nested dicts included, exactly like utils.stack_tensor_dict_list (meta_policy_search/utils/utils.py) of the unmodified
+    reference on the same seeded steps (tests/golden/stack_tensor_dict_list.npz)."""
     from promp_b200.samplers.meta_sampler import _stack
+    want = np.load(os.path.join(golden_dir, 'stack_tensor_dict_list.npz'))
     rng = np.random.RandomState(0)
     steps = [dict(mean=rng.randn(3), log_std=rng.randn(3), nested=dict(a=rng.randn(2), b=float(i))) for i in range(7)]
-    want, got = ref_utils.stack_tensor_dict_list(steps), _stack(steps)
-    assert set(want) == set(got) and set(want['nested']) == set(got['nested'])
+    got = _stack(steps)
+    assert sorted(got) == list(want['keys']) and sorted(got['nested']) == list(want['nested_keys'])
     for k in ('mean', 'log_std'):
         np.testing.assert_array_equal(got[k], want[k])
     for k in ('a', 'b'):
-        np.testing.assert_array_equal(got['nested'][k], want['nested'][k])
+        np.testing.assert_array_equal(got['nested'][k], want['nested_' + k])
     assert _stack([]) == {} and _stack([{}, {}]) == {}
 
 
